@@ -2,7 +2,7 @@
 """Benchmark of the plane-sweep cost-volume hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg2|cfg1|cfg3|cfg4|stress_dot|stress_hero] [--no-also]
+                    [--workload cfg2|cfg1|cfg3|cfg4|stress_dot|stress_hero] [--no-also] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic frame tuples: one
 ``FeatureVolumeManager.forward`` (hero, metadata-MLP matching) or ``CostVolumeManager.forward``
@@ -27,9 +27,13 @@ Prints ONE JSON line (rank 0).  Keys beyond the base contract:
   e2e           same metric through the public manager API with HOST (pinned) inputs
                 and outputs: H2D + sweep + D2H inside the timed region; median of 3 windows
 `--impl reference` times the CPU port alone on the SAME config (the reference is pure
-Python/PyTorch and /root/reference does not travel to the GPU box; the port is op-for-op the
-reference's own sequence and is pinned bit-exact against it in tests/test_oracle_vs_reference.py);
+Python/PyTorch and not part of this repository; the port is op-for-op the reference's own sequence
+and is pinned against its recorded outputs in tests/test_oracle_vs_reference.py);
 each step is a bounded sample of the batch (stated in `cpu_baseline.sample`), the metric is per frame.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<workload>_<output>.npy,
+float32, so that two builds can be compared output for output: the inputs are seeded and depend only
+on the arguments.  Past 64 MB in all, each array is replaced by a fixed seeded sample of its flattened
+elements (the same sample for the same shape).
 """
 from __future__ import annotations
 
@@ -52,6 +56,8 @@ import torch  # noqa: E402
 METRIC = "cost_volume_frames_per_sec@640x480_D64_K7src"
 UNIT = "frames/s"
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 64 * 10**6
+OUTPUT_NAMES = ("cost_volume", "lowest_cost", "depth_planes", "overall_mask")
 DEFAULT_WORKLOAD = "cfg2"
 ALSO_WORKLOAD = "cfg1"
 # frames per GPU (weak scaling): the single-GPU configuration's batch
@@ -378,7 +384,8 @@ def run_reference_arm(args, w, per_gpu):
 # GPU arm                                                                     #
 # --------------------------------------------------------------------------- #
 def measure_gpu(w, per_gpu, steps, warmup, dev, rank, world, sampler, S, _native, sharding, variant_id):
-    """value (device-resident inputs), the sweep kernel alone (roofline), and e2e (host buffers)."""
+    """value (device-resident inputs), the sweep kernel alone (roofline), and e2e (host buffers);
+    `outputs`: what the last timed step returned, on the host."""
     from simplerecon_b200.pipeline import HostStreamer
     from simplerecon_b200.synthetic import make_workload_tuple, mlp_state
     hero = w.kind == "mlp"
@@ -412,8 +419,9 @@ def measure_gpu(w, per_gpu, steps, warmup, dev, rank, world, sampler, S, _native
         torch.cuda.synchronize()
         sampler.active.set()
         e0.record()
-        for i in range(steps):
+        for i in range(steps - 1):
             step(i)
+        last = step(steps - 1)
         e1.record()
         torch.cuda.synchronize()
         sampler.active.clear()
@@ -457,7 +465,14 @@ def measure_gpu(w, per_gpu, steps, warmup, dev, rank, world, sampler, S, _native
             # larger so host-side stalls are not hidden
             windows.append(sharding.max_over_ranks(max(e0.elapsed_time(e1), 1e3 * t_wall), dev))
         e2e_ms = statistics.median(windows)
-    del sets_dev, pin, streamer, mgr
+    outputs = {}
+    for name, t in zip(OUTPUT_NAMES, last):
+        if t is None:
+            continue
+        if name == "depth_planes" and t.stride()[2:] == (0, 0):
+            t = t[:, :, :1, :1]          # one depth per plane, broadcast over the map: (B, D, 1, 1)
+        outputs[name] = t.float().cpu()
+    del sets_dev, pin, streamer, mgr, last
     torch.cuda.empty_cache()
 
     frames_step = per_gpu * world
@@ -471,9 +486,30 @@ def measure_gpu(w, per_gpu, steps, warmup, dev, rank, world, sampler, S, _native
                 "windows_ms_per_step": [x / e2e_steps for x in windows],
                 "mode": ("HostStreamer: H2D(i+1) || sweep(i) || D2H(i-1) on three streams, pinned host buffers, "
                          "persistent device input ring; median of 3 windows")},
-        "gpu_launches": launches, "clocks": clocks, "kernel_variant": variant,
+        "gpu_launches": launches, "clocks": clocks, "kernel_variant": variant, "outputs": outputs,
     }
     return rec
+
+
+def dump_outputs(directory: str, arrays: dict) -> dict:
+    """Writes `arrays` as <name>.npy (float32); past DUMP_BYTES in all, each array becomes a seeded
+    sample of its flattened elements, sorted by position.  Returns {name: shape, or the sample size}."""
+    import numpy as np
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    total = sum(4 * t.numel() for t in arrays.values())
+    frac = min(1.0, DUMP_BYTES / total) if total else 1.0
+    written = {}
+    for name, t in arrays.items():
+        a = t.numpy().astype(np.float32, copy=False)
+        if frac < 1.0:
+            idx = np.random.default_rng(0).choice(a.size, max(1, int(a.size * frac)), replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+            written[name] = f"seeded sample of {a.size} of {t.numel()} elements of {list(t.shape)}"
+        else:
+            written[name] = list(t.shape)
+        np.save(out / f"{name}.npy", a)
+    return written
 
 
 def main():
@@ -486,8 +522,12 @@ def main():
     ap.add_argument("--variant", default="auto", choices=["auto", "generic", "fast"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the secondary (dot cfg1) record")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of each workload to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     from simplerecon_b200.synthetic import CONFIGS, STRESS, mlp_state
     w = next(c for c in CONFIGS + STRESS if c.name.startswith(args.workload))
@@ -531,6 +571,11 @@ def main():
         line["also"] = {wa.name: {k: ra[k] for k in ("value", "ms_per_step", "config", "roofline", "e2e",
                                                      "gpu_launches", "clocks", "kernel_variant")}}
     sampler.stop()
+    if rank == 0 and args.dump_outputs:
+        dumped = {f"{w.name.split('_')[0]}_{k}": v for k, v in rec["outputs"].items()}
+        if "also" in line:
+            dumped.update({f"{wa.name.split('_')[0]}_{k}": v for k, v in ra["outputs"].items()})
+        line["dumped_outputs"] = {"dir": args.dump_outputs, "arrays": dump_outputs(args.dump_outputs, dumped)}
 
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         if full_affinity is not None:

@@ -12,9 +12,8 @@ cost volume + image-prior features into the depth map.  They live only in /root/
     python scripts/depth_parity.py eval        ->  profiles/depth_parity_r02.json
 
 Round 2: a BATCH per model — 8 hero frames (one B = 8 call, BASELINE configs[2]'s shard) and 4
-dot frames (configs[1]) at 640x480 — with the Abs-Diff reported per frame.  The two halves are
-also tests: tests/test_gpu_depth_parity.py writes the dump on the GPU box, tests/test_depth_parity_eval.py
-evaluates it here when both the dump and /root/reference are present.
+dot frames (configs[1]) at 640x480 — with the Abs-Diff reported per frame.  tests/test_gpu_depth_parity.py
+runs the first half (into a temporary directory) and checks the dump's shapes and kernel variants.
 
 Seeded random weights everywhere (no checkpoint exists in this environment, SURVEY.md §8c);
 image-prior pyramid = seeded random tensors with EfficientNetV2-S channel counts
@@ -42,7 +41,7 @@ DUMP = ROOT / "gpurun_out" / "depth_parity_ours.npz"
 REPORT = ROOT / "profiles" / "depth_parity_r02.json"
 
 
-def dump():
+def dump(path: Path = DUMP):
     import simplerecon_b200 as S
     from simplerecon_b200 import _native
     from simplerecon_b200.synthetic import to_device
@@ -60,9 +59,9 @@ def dump():
             out[f"{kind}_cost"] = cost.cpu().numpy()
             out[f"{kind}_lowest"] = lowest.cpu().numpy()
             out[f"{kind}_variant"] = np.array(_native.last_variant())
-    DUMP.parent.mkdir(exist_ok=True)
-    np.savez_compressed(DUMP, **out)
-    print("wrote", DUMP, {k: getattr(v, "shape", None) for k, v in out.items()})
+    path.parent.mkdir(exist_ok=True)
+    np.savez_compressed(path, **out)
+    print("wrote", path, {k: getattr(v, "shape", None) for k, v in out.items()})
 
 
 def evaluate(write: bool = True) -> dict:

@@ -53,7 +53,8 @@ def run_case(R, name, kind, tup, D, mlp_sd=None, depth_planes=None, return_mask=
     out = {k: tup[k].numpy() for k in INPUT_KEYS}
     out.update(kind=np.array(kind), D=np.array(D), ref_cost=cost.numpy(), ref_lowest=lowest.numpy(),
                ref_planes=planes[:, :, 0, 0].numpy() if depth_planes is None else planes.contiguous().numpy(),
-               ref_cost64=cost64.numpy(), ref_lowest64=lowest64.numpy())
+               ref_cost64_minus_ref_cost=(cost64 - cost.double()).float().numpy(),  # keeps files < 1 MB
+               ref_lowest64=lowest64.numpy())
     if depth_planes is not None:
         out["depth_planes_bdhw"] = depth_planes.contiguous().numpy()
     if mask is not None:

@@ -41,6 +41,8 @@ def load_golden(name):
          for k in z.files}
     g["kind"] = str(z["kind"])
     g["D"] = int(z["D"])
+    if "ref_cost64_minus_ref_cost" in g:     # stored as an fp32 residual where the fp64 volume is large
+        g["ref_cost64"] = g["ref_cost"].double() + g.pop("ref_cost64_minus_ref_cost").double()
     inputs = {k: g[k] for k in INPUT_KEYS}
     if "depth_planes_bdhw" in g:
         inputs["depth_planes_bdhw"] = g["depth_planes_bdhw"]
@@ -78,6 +80,13 @@ def load_golden_fullsize(name):
         g["ref_mask"] = torch.from_numpy(z["ref_mask"])
     sd = mlp_state(gen["views"], gen["channels"], seed=gen["seed"]) if g["kind"] == "mlp" else None
     return g, inputs, sd
+
+
+def load_reference_outputs(name):
+    """What the unmodified reference computed for the cases of one test module
+    (tests/golden/make_golden_reference.py), as CPU tensors; string arrays stay numpy."""
+    z = np.load(GOLDEN / "reference" / f"{name}.npz")
+    return {k: (z[k] if z[k].dtype.kind == "U" else torch.from_numpy(z[k])) for k in z.files}
 
 
 def cost_tol(kind, ref):

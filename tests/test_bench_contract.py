@@ -5,6 +5,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import pytest
+
 ROOT = Path(__file__).resolve().parents[1]
 
 
@@ -61,3 +63,48 @@ def test_mlp_flops_match_survey_and_configs_agree_between_arms():
     w = next(c for c in CONFIGS if c.name.startswith(bench.DEFAULT_WORKLOAD))
     c1, _ = bench.workload_config(w, bench.PER_GPU["cfg2"], 8)
     assert c1["global_batch"] == 64 and c1["matching"] == "mlp" and c1["planes"] == 64
+
+
+def test_dump_outputs_samples_past_the_budget(tmp_path, monkeypatch):
+    """Under the budget every array is written whole; past it each becomes the same seeded sample."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, str(ROOT))
+    import bench
+    a = torch.arange(6000, dtype=torch.float32).reshape(2, 3000)
+    b = torch.ones(4, 5, dtype=torch.float64)
+    info = bench.dump_outputs(str(tmp_path / "whole"), {"a": a, "b": b})
+    assert info == {"a": [2, 3000], "b": [4, 5]}
+    assert np.array_equal(np.load(tmp_path / "whole" / "a.npy"), a.numpy())
+    assert np.load(tmp_path / "whole" / "b.npy").dtype == np.float32
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4 * 1200)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"a": a})
+    s1, s2 = np.load(tmp_path / "s1" / "a.npy"), np.load(tmp_path / "s2" / "a.npy")
+    assert s1.shape == (1200,) and np.array_equal(s1, s2)
+    assert np.all(np.diff(s1) > 0)                      # distinct elements, in storage order
+
+
+@pytest.mark.gpu
+def test_dump_outputs_holds_the_last_timed_step(tmp_path):
+    """`--dump-outputs` writes what the last of `--steps` timed steps returned: its input set is the
+    seeded tuple of that step, so the dump equals the oracle's volume for that tuple."""
+    import numpy as np
+    sys.path.insert(0, str(ROOT))
+    from oracle import costvolume_oracle as O
+    from simplerecon_b200.synthetic import CONFIGS, make_workload_tuple
+    steps = 3
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "cfg0", "--steps", str(steps),
+                        "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps and set(line["dumped_outputs"]["arrays"]) == {
+        "cfg0_cost_volume", "cfg0_lowest_cost", "cfg0_depth_planes"}
+    w = CONFIGS[0]
+    t = make_workload_tuple(w, seed_offset=steps - 1, batch=1)       # sets rotate: step i uses set i
+    oc, ol, op, _ = O.forward_dot(**t, num_depth_bins=w.planes)
+    cost = np.load(tmp_path / "cfg0_cost_volume.npy")
+    assert cost.dtype == np.float32 and cost.shape == tuple(oc.shape)
+    assert np.abs(cost - oc.numpy()).max() <= 4e-5 * float(oc.abs().max()) + 1e-6
+    assert np.load(tmp_path / "cfg0_depth_planes.npy").shape == (1, w.planes, 1, 1)

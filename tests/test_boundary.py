@@ -149,19 +149,31 @@ def test_synthetic_tuples_are_deterministic_and_shaped():
         ("mlp", 16, 7, 120, 160, 96), ("mlp", 64, 7, 120, 160, 64)]
 
 
-def test_install_against_the_real_reference_module():
-    """install() on the UNMODIFIED reference's modules.cost_volume (build container only): the
-    three names resolve to our classes, `isinstance` / `to_fast()` as used by test.py:196-198 keep
-    working, a state_dict produced by the reference class loads strictly into ours, and
-    uninstall() restores the reference."""
-    from oracle.ref_import import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("reference tree not mounted")
-    R = load_reference()
-    import modules.cost_volume as ref_cv          # importable once load_reference() put the tree on sys.path
-    orig = {n: getattr(ref_cv, n) for n in ("CostVolumeManager", "FeatureVolumeManager", "FastFeatureVolumeManager")}
-    ref_state = orig["FeatureVolumeManager"](12, 16, num_depth_bins=8, mlp_channels=[0, 128, 128, 1],
-                                             matching_dim_size=16, num_source_views=7).state_dict()
+def _reference_like_module(monkeypatch, name, class_names):
+    """A module under the reference's import name holding stand-ins for `class_names`, for install()."""
+    mod = types.ModuleType(name)
+    for n in class_names:
+        setattr(mod, n, type(n, (torch.nn.Module,), {}))
+    if "." in name:
+        pkg = types.ModuleType(name.split(".")[0])
+        pkg.__path__ = []
+        monkeypatch.setitem(sys.modules, pkg.__name__, pkg)
+    monkeypatch.setitem(sys.modules, name, mod)
+    monkeypatch.delitem(sys.modules, "experiment_modules.depth_model", raising=False)
+    return mod
+
+
+def test_install_against_the_real_reference_module(monkeypatch):
+    """install() on the reference's modules.cost_volume namespace: the three names resolve to our
+    classes, `isinstance` / `to_fast()` as used by test.py:196-198 keep working, the state_dict the
+    unmodified reference's FeatureVolumeManager produces (recorded by tests/golden/make_golden_reference.py)
+    loads strictly into ours, and uninstall() restores the reference's classes."""
+    from tests.parity import load_reference_outputs
+    R = load_reference_outputs("python_layer")
+    ref_state = {k[len("state_dict/"):]: v for k, v in R.items() if k.startswith("state_dict/")}
+    names = ("CostVolumeManager", "FeatureVolumeManager", "FastFeatureVolumeManager")
+    ref_cv = _reference_like_module(monkeypatch, "modules.cost_volume", names)
+    orig = {n: getattr(ref_cv, n) for n in names}
     try:
         patched = S.install()
         assert "modules.cost_volume" in patched
@@ -182,23 +194,20 @@ def test_install_against_the_real_reference_module():
         assert getattr(ref_cv, n) is c
 
 
-def test_install_swaps_the_real_reference_loss_class():
-    """install(losses=True) on the UNMODIFIED reference's losses module (build container only): MVDepthLoss
-    resolves to the kernel-backed mirror with the reference's constructor / forward / helper signatures;
-    uninstall() restores it."""
-    from oracle.ref_import import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("reference tree not mounted")
-    load_reference()
-    import importlib
-    ref_losses = importlib.import_module("losses")
+def test_install_swaps_the_real_reference_loss_class(monkeypatch):
+    """install(losses=True) on the reference's losses namespace: MVDepthLoss resolves to the kernel-backed
+    mirror, whose constructor / forward / helper signatures are those of the unmodified reference's
+    (recorded by tests/golden/make_golden_reference.py); uninstall() restores it."""
+    from tests.parity import load_reference_outputs
+    ref_sigs = {s.split()[0]: s.split()[1:] for s in load_reference_outputs("mvdepth_loss")["signatures"]}
+    _reference_like_module(monkeypatch, "modules.cost_volume", ())
+    ref_losses = _reference_like_module(monkeypatch, "losses", ("MVDepthLoss",))
     orig = ref_losses.MVDepthLoss
     try:
         patched = S.install(losses=True)
         assert "losses" in patched and ref_losses.MVDepthLoss is S.MVDepthLoss
         for name in ("__init__", "forward", "get_valid_mask", "get_error_for_pair"):
-            assert list(inspect.signature(getattr(S.MVDepthLoss, name)).parameters) == \
-                list(inspect.signature(getattr(orig, name)).parameters), name
+            assert list(inspect.signature(getattr(S.MVDepthLoss, name)).parameters) == ref_sigs[name], name
         loss = ref_losses.MVDepthLoss(192, 256)                     # depth_model.py:144-147
         assert loss.height == 192 and loss.width == 256
         with pytest.raises(RuntimeError):                           # CPU tensors: refused, no fallback

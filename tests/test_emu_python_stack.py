@@ -17,7 +17,7 @@ from oracle import costvolume_oracle as O
 from simplerecon_b200 import _native, cost_volume
 from simplerecon_b200.synthetic import make_tuple, mlp_state
 from tests import emu
-from tests.parity import assert_cost_close, assert_lowest_close, assert_mask_close
+from tests.parity import assert_cost_close, assert_lowest_close, assert_mask_close, load_reference_outputs
 
 
 @pytest.fixture()
@@ -235,7 +235,7 @@ def test_per_frame_depth_range_and_weight_image_cache(emulated):
 def test_fast_manager_warp_features_five_tuple(emulated):
     """FastFeatureVolumeManager.warp_features (reference modules/cost_volume.py:812-964): all planes
     at once, 5-tuple (world points, depths, warped, mask, pixel coordinates) — against the oracle,
-    and against the live reference class where /root/reference is mounted."""
+    and against the reference class's output (tests/golden/make_golden_reference.py)."""
     B, K, C, H, W, D = 2, 3, 8, 9, 12, 4
     t = make_tuple(B, K, H, W, channels=C, seed=31)
     m = _hero(K, C, H, W, D, fast=True)
@@ -255,17 +255,11 @@ def test_fast_manager_warp_features_five_tuple(emulated):
         assert torch.allclose(pix[:, :, d, 1].reshape(B, K, -1), py, rtol=0, atol=2e-4)
         assert torch.equal(mask[:, :, d].reshape(B, K, -1), (zp > 0).float())
         assert torch.allclose(world[:, 0, d, :3].reshape(B, 3, -1), X, rtol=1e-6, atol=1e-7)
-    from oracle.ref_import import load_reference, reference_available
-    if reference_available():
-        R = load_reference()
-        ref = R.FastFeatureVolumeManager(H, W, num_depth_bins=D)
-        uv_scale = torch.tensor([1.0 / W, 1.0 / H]).view(1, 1, 1, 2)
-        with torch.no_grad():
-            rw, rd, rf, rm, rp = ref.warp_features(t["src_feats"], t["src_extrinsics"], t["src_Ks"], t["cur_invK"],
-                                                   planes, B, K, C, uv_scale)
-        assert torch.allclose(world, rw, rtol=1e-6, atol=1e-7) and torch.equal(mask, rm)
-        assert torch.allclose(depths, rd, rtol=2e-6, atol=1e-6) and torch.allclose(pix, rp, rtol=0, atol=2e-4)
-        assert (warped - rf).abs().max().item() <= 4e-5 * rf.abs().max().item() + 1e-6
+    R = load_reference_outputs("python_layer")
+    rw, rd, rf, rm, rp = (R[f"warp_{k}"] for k in ("world", "depths", "feats", "mask", "pix"))
+    assert torch.allclose(world, rw, rtol=1e-6, atol=1e-7) and torch.equal(mask, rm)
+    assert torch.allclose(depths, rd, rtol=2e-6, atol=1e-6) and torch.allclose(pix, rp, rtol=0, atol=2e-4)
+    assert (warped - rf).abs().max().item() <= 4e-5 * rf.abs().max().item() + 1e-6
 
 
 def test_producer_side_fusion_chunk_planar_and_raw_poses(emulated):

@@ -1,46 +1,23 @@
-"""CPU, build container only: the multi-view consistency oracle against the LIVE reference
-process_depth (tools/torch_point_cloud_fusion.py), whose hard-wired .cuda() calls are made no-ops."""
-import importlib.util
-import os
-
+"""CPU: the multi-view consistency oracle against the reference's process_depth
+(tools/torch_point_cloud_fusion.py), as recorded from the unmodified reference by
+tests/golden/make_golden_reference.py."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import mvs_oracle as M
-from oracle.ref_import import reference_available, reference_root
 from simplerecon_b200.synthetic import make_mvs_scene
-
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not mounted")
-
-
-def _load_reference_fuser(monkeypatch):
-    import sys
-    import types
-    if "tqdm" not in sys.modules:
-        try:
-            import tqdm  # noqa: F401
-        except Exception:
-            m = types.ModuleType("tqdm")
-            m.tqdm = lambda x, **k: x
-            sys.modules["tqdm"] = m
-    spec = importlib.util.spec_from_file_location(
-        "_simplerecon_ref_pcfusion", os.path.join(reference_root(), "tools", "torch_point_cloud_fusion.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)      # process_depth hard-wires .cuda()
-    return mod
+from tests.parity import load_reference_outputs
 
 
 @pytest.mark.parametrize("seed,n,hw", [(1, 5, (24, 32)), (2, 9, (30, 40))])
-def test_process_depth_matches_live_reference(monkeypatch, seed, n, hw):
-    R = _load_reference_fuser(monkeypatch)
+def test_process_depth_matches_live_reference(seed, n, hw):
+    R = load_reference_outputs("mvs")
     sc = make_mvs_scene(seed=seed, frames=n, height=hw[0], width=hw[1])
     depths, images, P, K = sc["depths"], sc["images"], sc["cam_T_world"], sc["K"]
     for ref_idx in (0, n // 2):
         src = torch.arange(n) != ref_idx
-        rp, rrgb, rvalid = R.process_depth(depths[ref_idx], images[ref_idx], depths[src], images[src],
-                                           P[ref_idx], P[src], K[ref_idx], K[src], 0.1, 3)
+        rp, rrgb, rvalid = (R[f"s{seed}_r{ref_idx}_{k}"].numpy() for k in ("points", "rgb", "valid"))
         pts_avg, n_valid, valid = M.process_depth_dense(depths[ref_idx], depths[src], P[ref_idx], P[src],
                                                         K[ref_idx], K[src], 0.1, 3)
         assert np.array_equal(valid.numpy(), rvalid) and 0.05 < valid.float().mean().item() < 0.99
