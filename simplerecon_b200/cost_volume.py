@@ -500,18 +500,25 @@ class FeatureVolumeManager(CostVolumeManager):
         w = _native.MlpWeights(*[x.data_ptr() for x in ts], lin[0].out_features, lin[1].out_features, None)
         return w, ts
 
-    def _attach_packed_image(self, dev, shape, w, ts):
+    def _attach_packed_image(self, dev, shape, w):
         """Points ``w.packed_image`` at the tensor-core kernel's fp16 weight image, re-packing it
-        (``srcv_mlp_pack_weights``) only when a parameter changed: the cache key is every
-        parameter's (storage address, version counter).  Returns what must stay alive."""
+        (``srcv_mlp_pack_weights``) only when a parameter changed.  The cache key is, for every
+        ``weight`` / ``bias`` of the MLP's linear layers, the Parameter's identity, storage
+        address, version counter and dtype — of the parameters themselves, not of the fp32
+        copies ``_f32c`` makes of fp16 / bf16 weights, which are fresh tensors at version 0 on
+        every call.  So replacing a Parameter, ``load_state_dict``, an optimizer step or any
+        other in-place update re-packs, also under ``no_grad`` / ``inference_mode``.  Writes
+        through ``.data`` bypass the version counter and are not seen.  Returns what must
+        stay alive."""
         lib = _native.load()
         nbytes = lib.srcv_mlp_packed_bytes(C.byref(shape), C.byref(w))
         if nbytes == 0:
             return None                                   # SIMT variant: nothing to pack
+        params = [p for l in self.mlp.net if isinstance(l, nn.Linear) for p in (l.weight, l.bias)]
         try:
-            key = (str(dev), tuple((t.data_ptr(), t._version) for t in ts))
-        except RuntimeError:                              # inference tensors carry no version counter
-            key = None
+            key = (str(dev), tuple((id(p), p.data_ptr(), p._version, p.dtype) for p in params))
+        except RuntimeError:                              # parameters created under inference_mode
+            key = None                                    # carry no version counter: pack every call
         cache = self.__dict__.get("_srcv_packed")
         if key is None or cache is None or cache[0] != key:
             with torch.cuda.device(dev):
@@ -551,7 +558,7 @@ class FeatureVolumeManager(CostVolumeManager):
             max_depth, depth_planes_bdhw, need_poses=True, allow_grad=allow_grad, raw_poses=raw_poses)
         n_features = shape.C * (shape.K + 1) + 10 * shape.K + 4
         w, wkeep = self._mlp_weights(dev, n_features)
-        wkeep.append(self._attach_packed_image(dev, shape, w, wkeep))
+        wkeep.append(self._attach_packed_image(dev, shape, w))
         with torch.cuda.device(dev):
             cost = torch.empty(shape.B, shape.D, shape.H, shape.W, device=dev, dtype=torch.float32)
             lowest = torch.empty(shape.B, shape.H, shape.W, device=dev, dtype=torch.float32) \

@@ -333,6 +333,37 @@ def test_hero_cfg3_planes_96_and_batch_shards():
     assert_mask_close(mask[3:], om)
 
 
+def test_hero_at_the_reference_training_resolution():
+    """512x384 frames (the reference's default, options.py:70-71): the 96x128 feature map runs the
+    tensor-core kernel's <false, 128, 96> instantiation.  B = 2, D = 64, planes from the range;
+    frame 0 against the oracle on every ninth plane (ending with the last, whose mask is the
+    volume's), frame 1 alone against frame 1 in the batch, and the SIMT kernel against both."""
+    B, K, H, W, D = 2, 7, 96, 128, 64
+    t = make_tuple(B, K, H, W, seed=131)
+    sd = mlp_state(K, 16, seed=7)
+    (cost, lowest, planes, mask), used = run_gpu("mlp", t, D, sd, variant="fast")
+    assert "tc" in used and cost.shape == (B, D, H, W) and mask.shape == (B, H, W)
+    sub = list(range(0, D, 9))
+    assert sub[-1] == D - 1
+    t0 = {k: (v[:1] if v.dim() > 0 and v.shape[0] == B else v) for k, v in t.items()}
+    p0 = planes[:1, sub].cpu().contiguous()
+    wts = O.mlp_weights_from_state_dict(sd)
+    oc, _, _, om = O.forward_mlp(**t0, weights=wts, num_depth_bins=len(sub), depth_planes_bdhw=p0, return_mask=True)
+    oc64, *_ = O.forward_mlp(**{k: v.double() for k, v in t0.items()}, weights=tuple(x.double() for x in wts),
+                             num_depth_bins=len(sub), depth_planes_bdhw=p0.double())
+    assert_cost_close("mlp", cost[:1, sub], oc, oc64, what="96x128 frame 0")
+    assert_mask_close(mask[:1], om)
+    idx = cost.argmax(1, keepdim=True)
+    assert torch.equal(torch.gather(planes.expand_as(cost), 1, idx).squeeze(1), lowest)
+    t1 = {k: (v[1:] if v.dim() > 0 and v.shape[0] == B else v) for k, v in t.items()}
+    (cost1, lowest1, _, mask1), _ = run_gpu("mlp", t1, D, sd, variant="fast")
+    assert torch.equal(cost1, cost[1:]) and torch.equal(lowest1, lowest[1:]) and torch.equal(mask1, mask[1:])
+    (cost_g, lowest_g, _, mask_g), used_g = run_gpu("mlp", t, D, sd, variant="generic")
+    assert "generic" in used_g and torch.equal(mask_g, mask)
+    assert (cost_g - cost).abs().max().item() <= cost_tol("mlp", oc)
+    assert_lowest_close("mlp", lowest, planes, cost_g.cpu(), what="96x128 lowest vs the SIMT volume")
+
+
 def test_bench_gpu_arm_prints_one_json_line():
     """bench.py (ours, N=1, default workload): stdout is exactly ONE JSON line with the contract's
     keys, kernels were launched, and the roofline / e2e / clock blocks are populated."""
@@ -372,6 +403,10 @@ def test_bench_gpu_arm_prints_one_json_line():
     (2, 3, 16, 14, 18, 5, 71, False),
     (1, 7, 16, 24, 32, 8, 72, False),
     (1, 2, 8, 10, 12, 4, 73, True),
+    (2, 7, 16, 96, 128, 8, 74, True),      # fast forward at its 512x384-frame size, C = 16 per-pixel backward
+    (1, 7, 16, 120, 160, 4, 75, True),
+    (1, 3, 32, 11, 13, 4, 76, False),      # C = 32 (generic forward), both plane modes
+    (2, 3, 32, 11, 13, 3, 77, True),
 ])
 def test_dot_backward_matches_autograd_of_the_oracle(B, K, C, H, W, D, seed, per_pixel):
     """Training path of CostVolumeManager: dL/dcur_feats and dL/dsrc_feats from the backward
@@ -394,6 +429,7 @@ def test_dot_backward_matches_autograd_of_the_oracle(B, K, C, H, W, D, seed, per
     m = make_manager("dot", K, C, H, W, D)
     cost, lowest, planes_ret, mask = m(**d, depth_planes_bdhw=planes.cuda() if per_pixel else None)
     assert cost.requires_grad and not lowest.requires_grad and mask is None
+    assert _native.last_variant() == ("dot_fast_c4planar" if C == 16 else "dot_generic")
     assert_cost_close("dot", cost, oc.detach())
     (cost * gcost.cuda()).sum().backward()
     assert _native.last_variant() == "dot_backward_atomic"
@@ -433,12 +469,15 @@ def _edge_views(t):
     return t
 
 
-@pytest.mark.parametrize("variant", ["generic", "fast"])
-def test_hero_k7_edge_views_and_per_pixel_planes(variant):
+@pytest.mark.parametrize("variant,H,W", [
+    pytest.param(v, H, W, id=v if (H, W) == (19, 27) else f"{v}-{H}x{W}")
+    for H, W in [(19, 27), (96, 128), (120, 160)] for v in ("generic", "fast")])
+def test_hero_k7_edge_views_and_per_pixel_planes(variant, H, W):
     """The tensor-core kernel (and the SIMT one) on the reference's corner cases at the hero
     layout: behind-camera and out-of-frustum source views, caller-supplied per-pixel depth
-    hypotheses (including a non-positive one), partial tiles."""
-    B, K, H, W, D = 1, 7, 19, 27, 4
+    hypotheses (including a non-positive one), partial tiles — at a generic map size and at both
+    sizes the tensor-core kernel is instantiated for (512x384 and 640x480 frames)."""
+    B, K, D = 1, 7, 4
     t = _edge_views(make_tuple(B, K, H, W, seed=81))
     sd = mlp_state(K, 16, seed=5)
     g = torch.Generator().manual_seed(82)

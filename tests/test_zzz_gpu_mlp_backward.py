@@ -65,6 +65,9 @@ def _oracle_grads(t, wts, D, gcost, planes, dtype=torch.float64):
     (1, 7, 16, 16, 20, 4, (128, 128), False, False),   # hero layout: tcgen05 forward, fp32 recompute backward
     (2, 2, 8, 13, 17, 3, (128, 128), True, False),     # generic forward, per-pixel planes, ragged tiles
     (1, 3, 16, 12, 16, 5, (96, 64), False, True),      # narrow hidden layers, Fast manager class
+    (1, 7, 16, 13, 17, 3, (128, 128), True, False),    # 202 input features per-pixel: backward <true, 13>
+    (1, 3, 16, 12, 16, 4, (96, 64), True, False),      # 98 input features per-pixel: backward <true, 8>
+    (1, 7, 16, 96, 128, 8, (128, 128), False, False),  # 512x384 frames: tcgen05 forward <false, 128, 96>
 ])
 def test_hero_training_matches_oracle_autograd(cuda_device, B, K, C, H, W, D, hidden, per_pixel, fast):
     t = make_tuple(B, K, H, W, channels=C, seed=31)
@@ -78,6 +81,8 @@ def test_hero_training_matches_oracle_autograd(cuda_device, B, K, C, H, W, D, hi
     cost, lowest, planes_ret, mask = m(**d, depth_planes_bdhw=planes.cuda() if per_pixel else None,
                                        return_mask=True)
     assert cost.requires_grad and not lowest.requires_grad and mask.dtype == torch.bool
+    hero = (K, C, tuple(hidden)) == (7, 16, (128, 128))
+    assert _native.last_variant() == ("mlp_tc_tcgen05_f16x3" if hero else "mlp_generic_fp32")
     (cost * gcost.cuda()).sum().backward()
     torch.cuda.synchronize()
     assert _native.last_variant() == "mlp_backward_fp32_recompute"
