@@ -293,6 +293,39 @@ size_t srcv_tsdf_workspace_bytes(const srcv_tsdf_frames* frames);
 int32_t srcv_tsdf_integrate_f16(const srcv_tsdf_volume* volume, const srcv_tsdf_frames* frames,
                                 void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- marching-cubes mesh extraction from the fused volume ---------------------------- *
+ * Replaces the host half of TSDF.to_mesh (reference tools/tsdf.py:125-157: a copy of the volume
+ * to the host and scikit-image's marching_cubes(level=0, allow_degenerate=False)).  Reads
+ * tsdf_values in place, clamped to [-1, 1] in fp32; a corner is below iff its value is < 0.
+ * Triangles whose vertices coincide in fp32 are dropped; with single_mesh, so is every triangle
+ * that needs a vertex on an edge from exactly -1 to exactly +1 (the boundary between observed free
+ * space and never-observed voxels).  Output in voxel-index space (axis 0, 1, 2):
+ *   verts, normals (V,3) fp32: one vertex per crossing edge a kept triangle uses, ordered by the
+ *                   owning voxel's linear index, then axis; normals = the normalised, linearly
+ *                   interpolated central-difference gradient (toward increasing values)
+ *   faces (F,3) int32: ordered by cell, then table order; counter-clockwise seen from above
+ * Two calls, two host synchronisations:
+ *   1. srcv_mesh_count_f16 writes counts[0] = candidate vertices, counts[1] = F, and counts[2] bit 0 /
+ *      bit 1 = the volume has a value >= 0 / <= 0 (level 0 inside [min, max] iff both are set);
+ *   2. the caller reads them, allocates faces (F,3) and verts / normals with room for counts[0]
+ *      rows, and srcv_mesh_emit_f16 (same volume, same workspace, untouched in between) writes
+ *      them and counts[3] = V <= counts[0]: rows V.. of verts / normals are unused.
+ * counts: DEVICE int64[4], 8-byte aligned.  Candidate and face counts must fit int32.
+ * scratch: DEVICE, srcv_mesh_scratch_bytes(counts[0]) bytes, 256-byte aligned.               */
+typedef struct srcv_mesh_volume {
+  const void* tsdf_values; /* DEVICE (X,Y,Z) fp16, z fastest, 2-byte aligned               */
+  int32_t X, Y, Z;         /* each >= 2                                                    */
+  int32_t single_mesh;     /* 0 / 1                                                        */
+} srcv_mesh_volume;
+size_t srcv_mesh_workspace_bytes(const srcv_mesh_volume* volume);
+size_t srcv_mesh_scratch_bytes(int32_t n_candidates);
+int32_t srcv_mesh_count_f16(const srcv_mesh_volume* volume, int64_t* counts, void* workspace,
+                            size_t workspace_bytes, void* stream);
+int32_t srcv_mesh_emit_f16(const srcv_mesh_volume* volume, int32_t n_candidates, int32_t n_faces,
+                           float* verts, float* normals, int32_t* faces, int64_t* counts,
+                           void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                           void* stream);
+
 /* ---- multi-view depth consistency (point-cloud fusion) ------------------------------ *
  * Replaces process_depth of the reference's 3DVNet-style fuser (tools/torch_point_cloud_fusion.py
  * :12-97), which pc_fusion.py:158 runs for every frame of a scan against all the others: for each

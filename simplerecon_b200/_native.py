@@ -66,6 +66,11 @@ class TsdfFrames(C.Structure):
                 ("H", C.c_int32), ("W", C.c_int32), ("min_depth", C.c_float), ("max_depth", C.c_float)]
 
 
+class MeshVolume(C.Structure):
+    _fields_ = [("tsdf_values", _fp), ("X", C.c_int32), ("Y", C.c_int32), ("Z", C.c_int32),
+                ("single_mesh", C.c_int32)]
+
+
 class MvsScan(C.Structure):
     _fields_ = [("depths", _fp), ("K", _fp), ("K_inv", _fp), ("cam_T_world", _fp), ("world_T_cam", _fp),
                 ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32)]
@@ -109,6 +114,11 @@ SYMBOLS = {
                                                       C.c_float, _fp, _fp, _fp]),
     "srcv_tsdf_workspace_bytes": (C.c_size_t, [C.POINTER(TsdfFrames)]),
     "srcv_tsdf_integrate_f16": (C.c_int32, [C.POINTER(TsdfVolume), C.POINTER(TsdfFrames), _fp, C.c_size_t, _fp]),
+    "srcv_mesh_workspace_bytes": (C.c_size_t, [C.POINTER(MeshVolume)]),
+    "srcv_mesh_scratch_bytes": (C.c_size_t, [C.c_int32]),
+    "srcv_mesh_count_f16": (C.c_int32, [C.POINTER(MeshVolume), _fp, _fp, C.c_size_t, _fp]),
+    "srcv_mesh_emit_f16": (C.c_int32, [C.POINTER(MeshVolume), C.c_int32, C.c_int32, _fp, _fp, _fp, _fp, _fp,
+                                       C.c_size_t, _fp, C.c_size_t, _fp]),
     "srcv_mvs_workspace_bytes": (C.c_size_t, [C.POINTER(MvsScan)]),
     "srcv_mvs_consistency_f32": (C.c_int32, [C.POINTER(MvsScan), C.c_int32, C.c_float, C.c_int32, _fp, _fp, _fp,
                                              _fp, C.c_size_t, C.c_int32, _fp]),

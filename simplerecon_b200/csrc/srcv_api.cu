@@ -455,6 +455,62 @@ int32_t srcv_tsdf_integrate_f16(const srcv_tsdf_volume* v, const srcv_tsdf_frame
   return SRCV_OK;
 }
 
+static int32_t check_mesh_volume(const srcv_mesh_volume* v) {
+  if (!v) return fail(SRCV_ERR_NULL, "mesh volume descriptor is NULL");
+  if (!v->tsdf_values) return fail(SRCV_ERR_NULL, "tsdf_values is NULL");
+  if (v->X < 2 || v->Y < 2 || v->Z < 2 || v->X >= (1 << 24) || v->Y >= (1 << 24) || v->Z >= (1 << 24) ||
+      (long long)v->X * v->Y > 2147483647ll || (long long)v->X * v->Y * v->Z > (1ll << 40))
+    return fail(SRCV_ERR_SHAPE, "bad mesh volume dimensions %d x %d x %d (each must be >= 2)", v->X, v->Y, v->Z);
+  if (v->single_mesh != 0 && v->single_mesh != 1) return fail(SRCV_ERR_SHAPE, "single_mesh must be 0 or 1");
+  if ((reinterpret_cast<uintptr_t>(v->tsdf_values) & 1u) != 0)
+    return fail(SRCV_ERR_UNSUPPORTED, "tsdf_values must be 2-byte aligned");
+  return SRCV_OK;
+}
+
+size_t srcv_mesh_workspace_bytes(const srcv_mesh_volume* v) {
+  if (!v || v->X < 2 || v->Y < 2 || v->Z < 2) return 0;
+  return mesh_workspace_bytes(*v);
+}
+
+size_t srcv_mesh_scratch_bytes(int32_t n_candidates) {
+  return n_candidates < 0 ? 0 : mesh_scratch_bytes(n_candidates);
+}
+
+int32_t srcv_mesh_count_f16(const srcv_mesh_volume* v, int64_t* counts, void* workspace, size_t workspace_bytes,
+                            void* stream_) {
+  if (int32_t e = check_mesh_volume(v)) return e;
+  if (!counts) return fail(SRCV_ERR_NULL, "counts is NULL");
+  if ((reinterpret_cast<uintptr_t>(counts) & 7u) != 0) return fail(SRCV_ERR_UNSUPPORTED, "counts must be 8-byte aligned");
+  if (int32_t e = check_workspace(workspace, workspace_bytes, mesh_workspace_bytes(*v))) return e;
+  g_last_variant.store("mesh_count_f16");
+  cudaError_t err = launch_mesh_count(*v, reinterpret_cast<long long*>(counts), workspace,
+                                      static_cast<cudaStream_t>(stream_));
+  if (err != cudaSuccess) return cuda_fail(err, "mesh_count");
+  return SRCV_OK;
+}
+
+int32_t srcv_mesh_emit_f16(const srcv_mesh_volume* v, int32_t n_candidates, int32_t n_faces, float* verts,
+                           float* normals, int32_t* faces, int64_t* counts, void* workspace, size_t workspace_bytes,
+                           void* scratch, size_t scratch_bytes, void* stream_) {
+  if (int32_t e = check_mesh_volume(v)) return e;
+  if (n_candidates < 0 || n_faces < 0 || n_faces > 2147483647 / 3)
+    return fail(SRCV_ERR_SHAPE, "bad counts: %d candidate vertices, %d faces (int32 overflow?)", n_candidates, n_faces);
+  if (!counts) return fail(SRCV_ERR_NULL, "counts is NULL");
+  if ((n_candidates > 0 && (!verts || !normals)) || (n_faces > 0 && !faces))
+    return fail(SRCV_ERR_NULL, "verts / normals / faces is NULL");
+  if (((reinterpret_cast<uintptr_t>(verts) | reinterpret_cast<uintptr_t>(normals) |
+        reinterpret_cast<uintptr_t>(faces)) & 3u) != 0 || (reinterpret_cast<uintptr_t>(counts) & 7u) != 0)
+    return fail(SRCV_ERR_UNSUPPORTED, "verts / normals / faces must be 4-byte aligned, counts 8-byte aligned");
+  if (int32_t e = check_workspace(workspace, workspace_bytes, mesh_workspace_bytes(*v))) return e;
+  if (int32_t e = check_workspace(scratch, scratch_bytes, mesh_scratch_bytes(n_candidates))) return e;
+  g_last_variant.store("mesh_emit_f16");
+  cudaError_t err = launch_mesh_emit(*v, n_candidates, n_faces, verts, normals, faces,
+                                     reinterpret_cast<long long*>(counts), workspace, scratch,
+                                     static_cast<cudaStream_t>(stream_));
+  if (err != cudaSuccess) return cuda_fail(err, "mesh_emit");
+  return SRCV_OK;
+}
+
 size_t srcv_mvs_workspace_bytes(const srcv_mvs_scan* s) {
   if (!s || s->N <= 0) return 0;
   return mvs_workspace_bytes(s->N);

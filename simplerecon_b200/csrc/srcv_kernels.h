@@ -103,6 +103,14 @@ size_t tsdf_workspace_bytes(int frames);
 cudaError_t launch_tsdf_integrate(const srcv_tsdf_volume& v, const srcv_tsdf_frames& f, void* workspace,
                                   cudaStream_t stream);
 
+// marching-cubes mesh extraction (csrc/srcv_mesh.cuh)
+size_t mesh_workspace_bytes(const srcv_mesh_volume& v);
+size_t mesh_scratch_bytes(long long n_candidates);
+cudaError_t launch_mesh_count(const srcv_mesh_volume& v, long long* counts, void* workspace, cudaStream_t stream);
+cudaError_t launch_mesh_emit(const srcv_mesh_volume& v, long long n_candidates, long long n_faces, float* verts,
+                             float* normals, int* faces, long long* counts, void* workspace, void* scratch,
+                             cudaStream_t stream);
+
 // multi-view depth consistency (csrc/srcv_mvs.cu)
 size_t mvs_workspace_bytes(int n);
 cudaError_t launch_mvs_consistency(const srcv_mvs_scan& s, int ref, float z_thresh, int n_consistent,

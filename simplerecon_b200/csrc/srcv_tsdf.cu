@@ -237,3 +237,6 @@ cudaError_t launch_tsdf_integrate(const srcv_tsdf_volume& v, const srcv_tsdf_fra
 }
 
 }  // namespace srcv
+
+// marching-cubes extraction from the same volume (TSDF.to_mesh)
+#include "srcv_mesh.cuh"
